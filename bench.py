@@ -2,10 +2,18 @@
 """bench.py -- audio-seconds/sec of the VSampler on the README U-Net (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg3|cfg5] [--impl reference]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one complete `model.sample(...)` call on each rank (weak scaling: the per-GPU batch is
 fixed, independent sampling, no collective on the data path).  Prints ONE JSON line (rank 0).
+K sets the timed steps of both sampling legs (device, e2e); the training leg is a separate
+measurement of a fixed 5 timed steps.
+
+--dump-outputs DIR writes rank 0's result of the last timed device step as DIR/sample.npy (float32,
+the whole [batch, 2, 2**18] clip: 16.8 MB for cfg2/cfg5, 33.6 MB for cfg3) and, when the training
+leg runs, the loss of its last timed step as DIR/train_loss.npy (float64).  Weights and inputs come
+from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
   --config cfg2 (default, BASELINE configs[1], the configuration `metric` is quoted on):
         unconditional README UNetV0, noise [8,2,2^18] per GPU, 50-step VSampler
@@ -35,6 +43,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -314,7 +323,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-ops", action="store_true", help="print the per-kernel table")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -369,8 +382,10 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
+    outputs = {}
+
     def step_device():
-        model.sample(dev_in, num_steps=num_steps, **dev_kw, **kw)
+        outputs["sample"] = model.sample(dev_in, num_steps=num_steps, **dev_kw, **kw)
 
     def step_e2e():
         x = host_in.to(dev, non_blocking=True)
@@ -383,6 +398,9 @@ def main():
         step_device()
     with ClockSampler(local) as clocks:
         total_ms = timed(step_device, args.steps)
+    last_sample = outputs.pop("sample")
+    dumps = {"sample": last_sample.float().cpu().numpy()} if args.dump_outputs else {}
+    del last_sample
     for _ in range(2):
         step_e2e()
     e2e_ms = timed(step_e2e, args.steps)
@@ -482,10 +500,15 @@ def main():
         gtab = table = None
         torch.cuda.empty_cache()
         line["train_step"] = train_step_bench(adp, dev, world, dist, steps=5, warmup=3)
+        dumps["train_loss"] = np.float64(line["train_step"]["loss"])
     if rank == 0 and not args.no_cpu_baseline and world == 1:
         v, per_step, cores, sample = cpu_reference_run(args.config, steps=1, warmup=1, budget_s=25.0, batch=1)
         line["cpu_baseline"] = {"value": v, "unit": "audio-s/s", "cores": cores, "kind": "port",
                                 "sample": sample}
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumps.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     if rank == 0:
         emit(json.dumps(line))
     if dist is not None:

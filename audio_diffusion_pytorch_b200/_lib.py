@@ -17,8 +17,7 @@ class ConvGemmArgs(C.Structure):
                 ("stats", vp), ("B", i32), ("T", i32), ("c_in", i32), ("lda", i32), ("ldo", i32),
                 ("k_total", i32), ("n_pad", i32), ("n_valid", i32), ("phases", i32),
                 ("ntaps", i32), ("tap_off", i32 * 3), ("up_factor", i32), ("groups", i32),
-                ("block_n", i32), ("out_fp32", i32), ("ld_gate", i32), ("gn_stats", vp),
-                ("gn_gamma", vp), ("gn_beta", vp), ("gn_eps", f32), ("gn_groups", i32)]
+                ("block_n", i32), ("out_fp32", i32), ("ld_gate", i32)]
 
 
 class StemInArgs(C.Structure):

@@ -56,32 +56,20 @@ inline cudaError_t ensure_dyn_smem(Kern kernel, size_t bytes, SmemAttrCache& cac
 // griddepcontrol.wait before its first global-memory access.  adp_debug_set(6, 0) disables.
 extern int g_pdl;
 template <typename Kern, typename... Args>
-inline cudaError_t launch_k_cluster(Kern kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                    int cluster_x, Args... args) {
+inline cudaError_t launch_k(Kern kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                            Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  if (cluster_x > 1) {       // thread-block cluster (CTA pairs of the tcgen05 cta_group::2 GEMM)
-    attr[1].id = cudaLaunchAttributeClusterDimension;
-    attr[1].val.clusterDim.x = static_cast<unsigned>(cluster_x);
-    attr[1].val.clusterDim.y = 1;
-    attr[1].val.clusterDim.z = 1;
-    cfg.numAttrs = 2;
-  }
   void* ptrs[] = {(void*)&args...};
   return cudaLaunchKernelExC(&cfg, (const void*)kernel, ptrs);
-}
-template <typename Kern, typename... Args>
-inline cudaError_t launch_k(Kern kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                            Args... args) {
-  return launch_k_cluster(kernel, grid, block, smem, st, 1, args...);
 }
 
 }  // namespace adp

@@ -24,11 +24,9 @@
 
 namespace adp {
 
-// diagnostic switches (adp_debug_set): [0] 3 = CTA-pair (cta_group::2) GEMMs; [2] 1 = weights are not
-// written by the preceding kernels (fetch them before griddepcontrol.wait); [3] CTAs/SM override;
-// [4] bit0 skip MMAs, bit1 skip TMA loads, bit2 skip drain, bit3 exit at entry (timing
-// experiments only); [5] KC override; [6] PDL; [7] 1 = never use the 8-epilogue-warp variant
-int g_debug[8] = {2, 1, 0, 0, 0, 0, 0, 0};
+// adp_debug_set(2, 1): the weights are not written by the preceding kernels, so the producer may
+// fetch them before griddepcontrol.wait (set while an inference graph is captured)
+int g_early_w = 0;
 
 constexpr int kBM = 128;
 constexpr int kMaxStages = 8;
@@ -51,31 +49,18 @@ struct Gemm2Params {
   int k_stages;          // stages per tile = (c_in / BK) / kc
   int n_stages;          // ring depth
   int a_sub_bytes, w_sub_bytes, stage_bytes, max_taps;
-  int dbg;
   int early_w;           // weights may be fetched before griddepcontrol.wait
-  // optional GroupNorm-apply + SiLU on the A operand (transform warps rewrite the smem tile)
-  const double* gn_stats;   // fp64 [B][gn_groups][2] of the A tensor
-  const float* gn_gamma;
-  const float* gn_beta;
-  float gn_eps;
-  int gn_groups;
 };
 
 struct TileInfo {
   int b, t0, n0, phase, ch0, ntaps, min_off;
-  bool valid;       // CTA pairs: the odd CTA of the last pair may have no rows
 };
 
-// cg = CTAs per tile (1, or 2 for cta_group::2 pairs: `tile` then indexes PAIR tiles of
-// 2*kBM rows and `rank` selects this CTA's 128 of them)
-__device__ __forceinline__ TileInfo tile_info(const Gemm2Params& p, int tile, int BN, int cg = 1,
-                                              int rank = 0) {
+__device__ __forceinline__ TileInfo tile_info(const Gemm2Params& p, int tile, int BN) {
   TileInfo ti;
-  const int m_pair = tile / p.n_tiles_n;
-  const int n_tile = tile - m_pair * p.n_tiles_n;
-  const int m_tile = m_pair * cg + rank;
+  const int m_tile = tile / p.n_tiles_n;
+  const int n_tile = tile - m_tile * p.n_tiles_n;
   ti.b = m_tile / p.tiles_per_batch;
-  ti.valid = ti.b < p.B;
   ti.t0 = (m_tile - ti.b * p.tiles_per_batch) * kBM;
   ti.n0 = n_tile * BN;
   ti.phase = ti.n0 / p.n_pad;
@@ -89,15 +74,6 @@ __device__ __forceinline__ TileInfo tile_info(const Gemm2Params& p, int tile, in
     ti.min_off = p.tap_off0;
   }
   return ti;
-}
-
-// SiLU with ONE special-function op per element (the transform warps are MUFU-bound):
-// z*sigmoid(z) = 0.5*z*(1 + tanh(z/2)); tanh.approx error (2^-11) is below bf16 rounding.
-__device__ __forceinline__ float silu_tanh(float z) {
-  float t;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * z));
-  const float hz = 0.5f * z;
-  return fmaf(hz, t, hz);
 }
 
 // thread-private GroupNorm partial sums: slot (value v of group g, epilogue thread et)
@@ -136,68 +112,50 @@ static __device__ __noinline__ void stats_generic(float* slots, int net, int et,
 // EW = epilogue warps: 4 (one per TMEM lane quarter) or, for the long-K shapes that run one CTA
 // per SM with <= one tile per CTA (nothing to overlap the drain with), 8: two warps per lane
 // quarter, each draining half of the tile's columns.
-// CG = 2: CTA PAIRS (cluster of 2 on one TPC, tcgen05 cta_group::2).  One MMA covers 256 rows x BN:
-// each CTA stages its own 128 rows of A but only HALF of the W tile, so the shared-memory fill
-// traffic per output drops from (A + W) to (A + W/2) per CTA -- the deep-level GEMMs are bound by
-// exactly that L2 -> SMEM traffic (profiles/r2_gemm_traffic.txt).  The leader (cluster rank 0)
-// issues every MMA and multicasts the completion to both CTAs' barriers; both CTAs run their own
-// TMA producer (signalling the LEADER's full barrier) and their own epilogue.
-template <int BN, int SW, bool XF, int EW, int CG = 1>
-__global__ void __launch_bounds__(64 + 32 * EW + (XF ? 256 : 0),
-                                  EW == 8 ? 1 : (BN <= 64 ? (XF ? 2 : 3) : (BN <= 128 ? (XF ? 1 : 2) : 1)))
+template <int BN, int SW, int EW>
+__global__ void __launch_bounds__(64 + 32 * EW, EW == 8 ? 1 : (BN <= 64 ? 3 : (BN <= 128 ? 2 : 1)))
 conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                   const Gemm2Params p) {
   constexpr int BK = SW / 2;
   constexpr int ACC_COLS = BN < 32 ? 32 : BN;     // TMEM columns per accumulator buffer
   constexpr int CH = BN < 32 ? 16 : 32;           // epilogue column chunk
-  constexpr int WN = BN / CG;                     // W rows staged by THIS CTA
-  constexpr uint32_t kWTapBytes = WN * SW;        // bytes one W box writes
-  static_assert(CG == 1 || (CG == 2 && !XF), "CTA pairs: plain (non-transform) variant only");
+  constexpr uint32_t kWTapBytes = BN * SW;        // bytes one W box writes
   extern __shared__ uint8_t smem_raw[];
-  __shared__ uint64_t full_bar[kMaxStages], empty_bar[kMaxStages], ready_bar[kMaxStages];
+  __shared__ uint64_t full_bar[kMaxStages], empty_bar[kMaxStages];
   __shared__ uint64_t acc_full[2], acc_empty[2];
   __shared__ uint32_t tmem_slot;
   constexpr int NET = 32 * EW;                    // epilogue threads
   constexpr int BNW = BN / (EW / 4);              // columns drained by one epilogue warp
-  static_assert(!XF || EW == 4, "the transform variant runs four epilogue warps");
   static_assert(EW == 4 || BNW >= 32, "8 epilogue warps need >= 32 columns per warp");
   __shared__ float s_part[2 * kMaxGroups * NET];
   // per-tile bias / gate of the BN output columns, double buffered like the accumulators:
   // staged while the tile's MMAs run so the drain never waits on a global load
   __shared__ __align__(16) float s_bias[2][BN < 32 ? 32 : BN];
   __shared__ __align__(16) float s_gate[2][BN < 32 ? 32 : BN];
-  __shared__ __align__(16) float s_coef[XF ? 2 * 1024 : 4];   // (a, d) per input channel of the current batch
 
   pdl_launch_dependents();
-  if (p.dbg & 8) return;      // timing experiment: launch floor of this configuration
   const int warp = warp_id_uniform();
   const int lane = threadIdx.x & 31;
   const uint32_t raw = smem_u32(smem_raw);
   uint8_t* ring = smem_raw + ((1024u - (raw & 1023u)) & 1023u);
 
-  const uint32_t rank = CG == 2 ? cluster_ctarank() : 0u;       // 0 = leader of the pair
-  const int tile_begin = (blockIdx.x / CG) * p.tiles_per_cta;
+  const int tile_begin = blockIdx.x * p.tiles_per_cta;
   int tile_end = tile_begin + p.tiles_per_cta;
   if (tile_end > p.total_tiles) tile_end = p.total_tiles;
 
   for (int i = threadIdx.x; i < 2 * kMaxGroups * NET; i += blockDim.x) s_part[i] = 0.f;
   if (warp == 0) {
-    if constexpr (CG == 2) { tmem_alloc_cg2(&tmem_slot, 2 * ACC_COLS); tmem_relinquish_cg2(); }
-    else { tmem_alloc(&tmem_slot, 2 * ACC_COLS); tmem_relinquish(); }
+    tmem_alloc(&tmem_slot, 2 * ACC_COLS);
+    tmem_relinquish();
   } else if (warp == 1 && lane == 0) {
-    // pairs: the leader's full barrier gets its own arrive.expect_tx plus the peer's remote arrive;
-    // the leader's acc_empty collects the epilogue warps of BOTH CTAs
-    for (int s = 0; s < p.n_stages; ++s) {
-      mbar_init(&full_bar[s], CG); mbar_init(&empty_bar[s], 1); mbar_init(&ready_bar[s], 256);
-    }
-    for (int s = 0; s < 2; ++s) { mbar_init(&acc_full[s], 1); mbar_init(&acc_empty[s], EW * CG); }
+    for (int s = 0; s < p.n_stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
+    for (int s = 0; s < 2; ++s) { mbar_init(&acc_full[s], 1); mbar_init(&acc_empty[s], EW); }
     fence_mbar_init();
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmW);
   }
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync_all();      // the peer's barriers exist before anyone signals them
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, tmem_slot, 0);   // warp-uniform for ptxas
   // Programmatic dependent launch: this kernel may have started while its predecessor still
@@ -212,27 +170,20 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       const uint32_t a_bytes = static_cast<uint32_t>(p.a_rows) * SW;
       const int total_it = (tile_end - tile_begin) * p.k_stages;
       int early = 0;
-      if (p.early_w && !(p.dbg & 2)) {
+      if (p.early_w) {
         early = total_it < p.n_stages ? total_it : p.n_stages;
         if (elect_one()) {
           int tile = tile_begin, ks = 0;
           for (int it = 0; it < early; ++it) {          // stage `it` of the (still empty) ring
-            const TileInfo ti = tile_info(p, tile, BN, CG, rank);
+            const TileInfo ti = tile_info(p, tile, BN);
             uint8_t* st = ring + it * p.stage_bytes;
             const uint32_t tx_it = static_cast<uint32_t>(p.kc) * (a_bytes + ti.ntaps * kWTapBytes);
-            const uint32_t lead_bar = CG == 2 ? mapa_shared(smem_u32(&full_bar[it]), 0) : 0u;
-            if (rank == 0) mbar_arrive_expect_tx(&full_bar[it], CG * tx_it);
-            else mbar_arrive_cluster(lead_bar);
+            mbar_arrive_expect_tx(&full_bar[it], tx_it);
             for (int c = 0; c < p.kc; ++c) {
               const int k0 = (ks * p.kc + c) * BK;
               uint8_t* wdst = st + p.kc * p.a_sub_bytes + c * p.max_taps * p.w_sub_bytes;
-              for (int tap = 0; tap < ti.ntaps; ++tap) {
-                if constexpr (CG == 2)
-                  tma_load_2d_cg2(wdst + tap * p.w_sub_bytes, &tmW, lead_bar, tap * p.c_in + k0,
-                                  ti.n0 + static_cast<int>(rank) * WN);
-                else
-                  tma_load_2d(wdst + tap * p.w_sub_bytes, &tmW, &full_bar[it], tap * p.c_in + k0, ti.n0);
-              }
+              for (int tap = 0; tap < ti.ntaps; ++tap)
+                tma_load_2d(wdst + tap * p.w_sub_bytes, &tmW, &full_bar[it], tap * p.c_in + k0, ti.n0);
             }
             if (++ks == p.k_stages) { ks = 0; ++tile; }
           }
@@ -243,38 +194,21 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       int s = 0, it = 0;
       uint32_t ph = 0;
       for (int tile = tile_begin; tile < tile_end; ++tile) {
-        const TileInfo ti = tile_info(p, tile, BN, CG, rank);
+        const TileInfo ti = tile_info(p, tile, BN);
         const uint32_t tx = static_cast<uint32_t>(p.kc) * (a_bytes + ti.ntaps * kWTapBytes);
         for (int ks = 0; ks < p.k_stages; ++ks, ++it) {
           const bool armed = it < early;                 // barrier armed + weights already issued
           if (!armed) mbar_wait(&empty_bar[s], ph ^ 1);
           uint8_t* st = ring + s * p.stage_bytes;
           if (elect_one()) {
-            const uint32_t lead_bar = CG == 2 ? mapa_shared(smem_u32(&full_bar[s]), 0) : 0u;
-            if (p.dbg & 2) {
-              if (rank == 0) mbar_arrive(&full_bar[s]);
-              else mbar_arrive_cluster(lead_bar);
-            } else {
-              if (!armed) {
-                if (rank == 0) mbar_arrive_expect_tx(&full_bar[s], CG * tx);
-                else mbar_arrive_cluster(lead_bar);
-              }
-              for (int c = 0; c < p.kc; ++c) {
-                const int k0 = (ks * p.kc + c) * BK;
-                if constexpr (CG == 2)
-                  tma_load_3d_cg2(st + c * p.a_sub_bytes, &tmA, lead_bar, k0, ti.t0 + ti.min_off, ti.b);
-                else
-                  tma_load_3d(st + c * p.a_sub_bytes, &tmA, &full_bar[s], k0, ti.t0 + ti.min_off, ti.b);
-                if (armed) continue;
-                uint8_t* wdst = st + p.kc * p.a_sub_bytes + c * p.max_taps * p.w_sub_bytes;
-                for (int tap = 0; tap < ti.ntaps; ++tap) {
-                  if constexpr (CG == 2)
-                    tma_load_2d_cg2(wdst + tap * p.w_sub_bytes, &tmW, lead_bar, tap * p.c_in + k0,
-                                    ti.n0 + static_cast<int>(rank) * WN);
-                  else
-                    tma_load_2d(wdst + tap * p.w_sub_bytes, &tmW, &full_bar[s], tap * p.c_in + k0, ti.n0);
-                }
-              }
+            if (!armed) mbar_arrive_expect_tx(&full_bar[s], tx);
+            for (int c = 0; c < p.kc; ++c) {
+              const int k0 = (ks * p.kc + c) * BK;
+              tma_load_3d(st + c * p.a_sub_bytes, &tmA, &full_bar[s], k0, ti.t0 + ti.min_off, ti.b);
+              if (armed) continue;
+              uint8_t* wdst = st + p.kc * p.a_sub_bytes + c * p.max_taps * p.w_sub_bytes;
+              for (int tap = 0; tap < ti.ntaps; ++tap)
+                tma_load_2d(wdst + tap * p.w_sub_bytes, &tmW, &full_bar[s], tap * p.c_in + k0, ti.n0);
             }
           }
           __syncwarp();
@@ -284,58 +218,45 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------------ MMA issuer
-    if (rank == 0) {       // pairs: the leader issues for both CTAs
-      constexpr uint32_t idesc = umma_idesc_bf16(kBM * CG, BN, 0, 0);
-      // descriptor of the ring base; byte offsets are added to the 14-bit address field
-      const uint64_t desc0 = umma_desc_kmajor<SW>(smem_u32(ring));
-      const uint32_t stage_u = static_cast<uint32_t>(p.stage_bytes) >> 4;
-      const uint32_t a_sub_u = static_cast<uint32_t>(p.a_sub_bytes) >> 4;
-      const uint32_t w_sub_u = static_cast<uint32_t>(p.w_sub_bytes) >> 4;
-      const uint32_t w_base_u = static_cast<uint32_t>(p.kc) * a_sub_u;
-      int s = 0;
-      uint32_t ph = 0, j = 0;
-      for (int tile = tile_begin; tile < tile_end; ++tile, ++j) {
-        const TileInfo ti = tile_info(p, tile, BN, CG, 0);
-        const uint32_t buf = j & 1;
-        mbar_wait(&acc_empty[buf], ((j >> 1) & 1) ^ 1);
+    constexpr uint32_t idesc = umma_idesc_bf16(kBM, BN, 0, 0);
+    // descriptor of the ring base; byte offsets are added to the 14-bit address field
+    const uint64_t desc0 = umma_desc_kmajor<SW>(smem_u32(ring));
+    const uint32_t stage_u = static_cast<uint32_t>(p.stage_bytes) >> 4;
+    const uint32_t a_sub_u = static_cast<uint32_t>(p.a_sub_bytes) >> 4;
+    const uint32_t w_sub_u = static_cast<uint32_t>(p.w_sub_bytes) >> 4;
+    const uint32_t w_base_u = static_cast<uint32_t>(p.kc) * a_sub_u;
+    int s = 0;
+    uint32_t ph = 0, j = 0;
+    for (int tile = tile_begin; tile < tile_end; ++tile, ++j) {
+      const TileInfo ti = tile_info(p, tile, BN);
+      const uint32_t buf = j & 1;
+      mbar_wait(&acc_empty[buf], ((j >> 1) & 1) ^ 1);
+      tc_fence_after();
+      const uint32_t d_tmem = tmem_base + buf * ACC_COLS;
+      uint32_t accumulate = 0;
+      for (int ks = 0; ks < p.k_stages; ++ks) {
+        mbar_wait(&full_bar[s], ph);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + buf * ACC_COLS;
-        uint32_t accumulate = 0;
-        for (int ks = 0; ks < p.k_stages; ++ks) {
-          mbar_wait(XF ? &ready_bar[s] : &full_bar[s], ph);
-          tc_fence_after();
-          if (elect_one()) {        // ONE elected thread issues the whole stage and its commit
-            if (!(p.dbg & 1)) {
-              const uint64_t sdesc = desc0 + static_cast<uint64_t>(s * stage_u);
-              for (int c = 0; c < p.kc; ++c) {
-                const uint64_t adesc = sdesc + c * a_sub_u;
-                const uint64_t wdesc = sdesc + w_base_u + c * p.max_taps * w_sub_u;
-                for (int tap = 0; tap < ti.ntaps; ++tap) {
+        if (elect_one()) {        // ONE elected thread issues the whole stage and its commit
+          const uint64_t sdesc = desc0 + static_cast<uint64_t>(s * stage_u);
+          for (int c = 0; c < p.kc; ++c) {
+            const uint64_t adesc = sdesc + c * a_sub_u;
+            const uint64_t wdesc = sdesc + w_base_u + c * p.max_taps * w_sub_u;
+            for (int tap = 0; tap < ti.ntaps; ++tap) {
 #pragma unroll
-                  for (int kk = 0; kk < BK / 16; ++kk) {
-                    if constexpr (CG == 2)
-                      umma_bf16_cg2(d_tmem, adesc + ((tap * SW + kk * 32) >> 4),
-                                    wdesc + tap * w_sub_u + ((kk * 32) >> 4), idesc, accumulate);
-                    else
-                      umma_bf16(d_tmem, adesc + ((tap * SW + kk * 32) >> 4),
-                                wdesc + tap * w_sub_u + ((kk * 32) >> 4), idesc, accumulate);
-                    accumulate = 1;
-                  }
-                }
+              for (int kk = 0; kk < BK / 16; ++kk) {
+                umma_bf16(d_tmem, adesc + ((tap * SW + kk * 32) >> 4),
+                          wdesc + tap * w_sub_u + ((kk * 32) >> 4), idesc, accumulate);
+                accumulate = 1;
               }
             }
-            if constexpr (CG == 2) {
-              umma_commit_cg2(&empty_bar[s], 3);
-              if (ks == p.k_stages - 1) umma_commit_cg2(&acc_full[buf], 3);
-            } else {
-              umma_commit(&empty_bar[s]);
-              if (ks == p.k_stages - 1) umma_commit(&acc_full[buf]);
-            }
           }
-          accumulate = 1;
-          __syncwarp();
-          if (++s == p.n_stages) { s = 0; ph ^= 1; }
+          umma_commit(&empty_bar[s]);
+          if (ks == p.k_stages - 1) umma_commit(&acc_full[buf]);
         }
+        accumulate = 1;
+        __syncwarp();
+        if (++s == p.n_stages) { s = 0; ph ^= 1; }
       }
     }
   } else if (warp < 2 + EW) {
@@ -371,13 +292,13 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     };
 
     for (int tile = tile_begin; tile < tile_end; ++tile, ++j) {
-      const TileInfo ti = tile_info(p, tile, BN, CG, rank);
+      const TileInfo ti = tile_info(p, tile, BN);
       const uint32_t buf = j & 1;
       const int t = ti.t0 + row;
-      const bool row_ok = t < p.T && ti.valid;
-      const size_t row_off = (static_cast<size_t>(ti.valid ? ti.b : 0) * p.T + (row_ok ? t : 0)) * p.ldo +
+      const bool row_ok = t < p.T;
+      const size_t row_off = (static_cast<size_t>(ti.b) * p.T + (row_ok ? t : 0)) * p.ldo +
                              static_cast<size_t>(ti.phase) * p.n_valid;
-      if (do_stats && ti.valid && ti.b != cur_b) {
+      if (do_stats && ti.b != cur_b) {
         if (cur_b >= 0) publish_stats(cur_b);
         cur_b = ti.b;
       }
@@ -396,7 +317,7 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         const int ch = ti.ch0 + c;
         const bool ok = ch < p.n_valid;
         s_bias[buf][c] = (p.bias && ok) ? __ldg(p.bias + ch) : 0.f;
-        s_gate[buf][c] = (p.gate && ok && ti.valid) ? __ldg(p.gate + static_cast<size_t>(ti.b) * p.ld_gate + ch) : 1.f;
+        s_gate[buf][c] = (p.gate && ok) ? __ldg(p.gate + static_cast<size_t>(ti.b) * p.ld_gate + ch) : 1.f;
       }
       named_bar_sync(2, NET);     // staging visible to all epilogue warps
       mbar_wait(&acc_full[buf], (j >> 1) & 1);
@@ -452,7 +373,7 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           }
         }
       };
-      const bool fast = !p.gate && !p.out_fp32 && !(p.dbg & 4) && ti.ch0 + cbeg + BNW <= p.n_valid &&
+      const bool fast = !p.gate && !p.out_fp32 && ti.ch0 + cbeg + BNW <= p.n_valid &&
                         (!do_stats || p.group_shift >= 3);
       if (fast) {
         if (p.residual) {
@@ -467,7 +388,6 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       for (int cc = 0; cc < BNW; cc += CH) {
         if (fast) break;
         const int c0 = cbeg + cc;
-        if (p.dbg & 4) break;   // timing experiment: skip the drain
         uint32_t r[CH];
         if constexpr (CH == 16) tmem_ld16(taddr + c0, r);
         else tmem_ld32(taddr + c0, r);
@@ -548,85 +468,16 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       // accumulator buffer drained -> hand it back to the MMA warp
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (CG == 2) mbar_arrive_cluster(mapa_shared(smem_u32(&acc_empty[buf]), 0));
-        else mbar_arrive(&acc_empty[buf]);
-      }
+      if (lane == 0) mbar_arrive(&acc_empty[buf]);
     }
     if (do_stats && cur_b >= 0) publish_stats(cur_b);
-  } else if constexpr (XF) {
-    // ------------------------------------------------- transform: a = silu(x*ga + de) in place
-    // 256 threads, two per tile row.  The TMA tile is SW-byte rows with the 16-byte chunks
-    // XOR-swizzled by address bits [7, 7+log2(SW/16)); zero rows (conv padding) stay zero.
-    pdl_wait();
-    const int tt = threadIdx.x - (64 + NET);
-    constexpr int CPR = SW / 16;                 // 16-byte chunks per row
-    constexpr int CPT = CPR / 2 > 0 ? CPR / 2 : 1;   // chunks per thread
-    const int gsz = p.c_in / p.gn_groups;
-    const double inv_n = 1.0 / (static_cast<double>(gsz) * p.T);
-    int s = 0, cur_b = -1;
-    uint32_t ph = 0;
-    for (int tile = tile_begin; tile < tile_end; ++tile) {
-      const TileInfo ti = tile_info(p, tile, BN);
-      if (ti.b != cur_b) {     // (a, d) of every input channel for this batch element, once
-        named_bar_sync(3, 256);          // previous batch's coefficients no longer in use
-        for (int ch = tt; ch < p.c_in; ch += 256) {
-          const int g = ch / gsz;
-          const double mean = p.gn_stats[(static_cast<size_t>(ti.b) * p.gn_groups + g) * 2] * inv_n;
-          const float var = fmaxf(static_cast<float>(
-              p.gn_stats[(static_cast<size_t>(ti.b) * p.gn_groups + g) * 2 + 1] * inv_n - mean * mean), 0.f);
-          const float ga = __ldg(p.gn_gamma + ch) * rsqrtf(var + p.gn_eps);
-          s_coef[2 * ch] = ga;
-          s_coef[2 * ch + 1] = __ldg(p.gn_beta + ch) - static_cast<float>(mean) * ga;
-        }
-        named_bar_sync(3, 256);
-        cur_b = ti.b;
-      }
-      for (int ks = 0; ks < p.k_stages; ++ks) {
-        mbar_wait(&full_bar[s], ph);
-        uint8_t* st = ring + s * p.stage_bytes;
-        for (int c = 0; c < p.kc; ++c) {
-          uint8_t* sub = st + c * p.a_sub_bytes;
-          const float* cf = s_coef + (ks * p.kc + c) * BK * 2;
-          for (int rr = tt >> 1; rr < p.a_rows; rr += 128) {
-            const int t = ti.t0 + ti.min_off + rr;
-            if (t < 0 || t >= p.T) continue;               // TMA zero fill = conv padding
-            const uint32_t row_off = static_cast<uint32_t>(rr) * SW;
-            const int swz = (row_off >> 7) & (CPR - 1);
-#pragma unroll
-            for (int q = 0; q < CPT; ++q) {
-              const int pc = (CPR >= 2) ? (tt & 1) * CPT + q : 0;      // physical chunk
-              if (CPR < 2 && (tt & 1)) continue;
-              const int lc = pc ^ swz;                                  // logical chunk
-              uint4* ptr = reinterpret_cast<uint4*>(sub + row_off + pc * 16);
-              const uint4 u = *ptr;
-              const float4* c4 = reinterpret_cast<const float4*>(cf + lc * 16);
-              const float4 k0 = c4[0], k1 = c4[1], k2 = c4[2], k3 = c4[3];   // (a,d) x 8 channels
-              const float2 f0 = unpack_bf16(u.x), f1 = unpack_bf16(u.y);
-              const float2 f2 = unpack_bf16(u.z), f3 = unpack_bf16(u.w);
-              uint4 o;
-              o.x = pack_bf16(silu_tanh(f0.x * k0.x + k0.y), silu_tanh(f0.y * k0.z + k0.w));
-              o.y = pack_bf16(silu_tanh(f1.x * k1.x + k1.y), silu_tanh(f1.y * k1.z + k1.w));
-              o.z = pack_bf16(silu_tanh(f2.x * k2.x + k2.y), silu_tanh(f2.y * k2.z + k2.w));
-              o.w = pack_bf16(silu_tanh(f3.x * k3.x + k3.y), silu_tanh(f3.y * k3.z + k3.w));
-              *ptr = o;
-            }
-          }
-        }
-        fence_proxy_async_smem();
-        mbar_arrive(&ready_bar[s]);
-        if (++s == p.n_stages) { s = 0; ph ^= 1; }
-      }
-    }
   }
 
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync_all();   // neither CTA's smem / TMEM / barriers may vanish early
-  else __syncthreads();
+  __syncthreads();
   if (warp == 0) {
     __syncwarp();
-    if constexpr (CG == 2) tmem_dealloc_cg2(tmem_base, 2 * ACC_COLS);
-    else tmem_dealloc(tmem_base, 2 * ACC_COLS);
+    tmem_dealloc(tmem_base, 2 * ACC_COLS);
   }
 }
 
@@ -641,40 +492,11 @@ static int num_sms() {
   return n;
 }
 
-template <int BN, int SW, bool XF, int EW, int CG = 1>
-static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int occ_in);
-
-// CTA pairs (cta_group::2) are OPT-IN: adp_debug_set(0, 3).  Measured on B200
-// (profiles/r2_gemm_pairs.txt): the pair MMA removes the shared-memory operand-read bound of the
-// 128 x 128 SS-MMA (MMA phase of the L7 conv3 5.5 us instead of 8.1 us), but every ring stage then
-// costs a cross-CTA handshake (multicast commit -> peer producer -> TMA -> leader's barrier,
-// ~1.8 us per round trip) that a 196 KB ring cannot hide: 16.6 us vs 16.2 us end to end.
-template <int BN, int SW, bool XF>
-static bool use_pairs(const adp_conv_gemm_args& a) {
-  if (BN != 128 || SW != 128 || XF || g_debug[0] != 3) return false;
-  const int taps = a.up_factor > 1 ? 2 : a.ntaps;
-  const long m_tiles = (long)a.B * ((a.T + kBM - 1) / kBM);
-  return m_tiles >= 2 && (a.c_in / 64) * taps >= 8;
-}
-
-template <int BN, int SW, bool XF>
+// EW = 4 picks the CTAs per SM from the shape and may hand over to the 8-drain-warp variant,
+// which always runs one CTA per SM.
+template <int BN, int SW, int EW = 4>
 static int launch_gemm2(const adp_conv_gemm_args& a, cudaStream_t stream) {
-  if constexpr (BN == 128 && SW == 128 && !XF) {
-    if (use_pairs<BN, SW, XF>(a)) {
-      const long m_pairs = ((long)a.B * ((a.T + kBM - 1) / kBM) + 1) / 2;
-      const long total = m_pairs * (a.phases * a.n_pad / BN);
-      // <= one pair tile per CTA pair: nothing overlaps the drain -> 8 drain warps
-      if (g_debug[7] == 0 && 2 * total <= 2L * num_sms()) return launch_gemm2_ew<BN, SW, XF, 8, 2>(a, stream, 1);
-      return launch_gemm2_ew<BN, SW, XF, 4, 2>(a, stream, 1);
-    }
-  }
-  return launch_gemm2_ew<BN, SW, XF, 4>(a, stream, 0);
-}
-
-template <int BN, int SW, bool XF, int EW, int CG>
-static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int occ_in) {
   constexpr int BK = SW / 2;
-  constexpr int WN = BN / CG;
   const int tiles_per_batch = (a.T + kBM - 1) / kBM;
   const bool up = a.up_factor > 1;
   const int max_taps = up ? 2 : a.ntaps;
@@ -684,31 +506,30 @@ static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int
 
   Gemm2Params p;
   p.a_sub_bytes = (a_rows * SW + 1023) / 1024 * 1024;
-  p.w_sub_bytes = (WN * SW + 1023) / 1024 * 1024;
+  p.w_sub_bytes = (BN * SW + 1023) / 1024 * 1024;
   p.max_taps = max_taps;
   const int chunk_bytes = p.a_sub_bytes + max_taps * p.w_sub_bytes;
 
+  auto budget_of = [](int o) {
+    return (o == 1 ? (EW == 8 ? 204 : 196) : (o == 2 ? 96 : 60)) * 1024;   // 227 KB - static - 1 KB
+  };  // <= 11 KB static smem/CTA
   // CTAs per SM: the epilogue (4 warps per CTA) is the critical resource of short-K tiles, so
   // those run 2-3 CTAs per SM; long-K tiles want deep rings of fat stages instead.
-  const int w_iters = k_chunks * max_taps;
   int occ = 1;
-  if (BN <= 64 && w_iters <= 8) occ = 3;
-  else if (BN <= 128 && w_iters <= 12) occ = 2;
-  if (XF && occ > (BN <= 64 ? 2 : 1)) occ = BN <= 64 ? 2 : 1;
-  if (g_debug[3] > 0) occ = g_debug[3];
-  if (occ_in > 0) occ = occ_in;
-  const int tmem_occ = 512 / (2 * (BN < 32 ? 32 : BN));
-  if (occ > tmem_occ) occ = tmem_occ;
-  auto budget_of = [](int o) {
-    return (o == 1 ? (EW == 8 ? 204 : 196) : (o == 2 ? (XF ? 92 : 96) : 60)) * 1024;   // 227 KB - static - 1 KB
-  };  // <= 11 KB static smem/CTA
-  while (occ > 1 && budget_of(occ) < 2 * chunk_bytes) --occ;   // need >= 2 stages in the ring
-  if constexpr (EW == 4 && !XF && BN >= 64 && CG == 1) {
-    // at most ~two tiles per SM: little or nothing overlaps the drain -> one CTA per SM with
-    // 8 drain warps (also when 2 CTAs/SM were possible but every SM gets <= one tile anyway)
-    const long total = (long)a.B * tiles_per_batch * (a.phases * a.n_pad / BN);
-    if (g_debug[7] == 0 && ((occ == 1 && total <= 2L * num_sms()) || total <= (long)num_sms()))
-      return launch_gemm2_ew<BN, SW, XF, 8>(a, stream, 1);
+  if constexpr (EW == 4) {
+    const int w_iters = k_chunks * max_taps;
+    if (BN <= 64 && w_iters <= 8) occ = 3;
+    else if (BN <= 128 && w_iters <= 12) occ = 2;
+    const int tmem_occ = 512 / (2 * (BN < 32 ? 32 : BN));
+    if (occ > tmem_occ) occ = tmem_occ;
+    while (occ > 1 && budget_of(occ) < 2 * chunk_bytes) --occ;   // need >= 2 stages in the ring
+    if constexpr (BN >= 64) {
+      // at most ~two tiles per SM: little or nothing overlaps the drain -> one CTA per SM with
+      // 8 drain warps (also when 2 CTAs/SM were possible but every SM gets <= one tile anyway)
+      const long total = (long)a.B * tiles_per_batch * (a.phases * a.n_pad / BN);
+      if ((occ == 1 && total <= 2L * num_sms()) || total <= (long)num_sms())
+        return launch_gemm2<BN, SW, 8>(a, stream);
+    }
   }
   const int budget = budget_of(occ);
   // chunks per stage: amortise one mbarrier round trip over >= 8 MMAs where smem allows
@@ -716,7 +537,6 @@ static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int
   while (kc * 2 <= 4 && k_chunks % (kc * 2) == 0 && kc * max_taps * (BK / 16) < 8 &&
          2 * (kc * 2) * chunk_bytes <= budget)
     kc *= 2;
-  if (g_debug[5] > 0 && k_chunks % g_debug[5] == 0) kc = g_debug[5];
   p.kc = kc;
   p.k_stages = k_chunks / kc;
   p.stage_bytes = kc * chunk_bytes;
@@ -737,12 +557,12 @@ static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int
   {
     const uint64_t dims[2] = {(uint64_t)a.k_total, (uint64_t)a.phases * a.n_pad};
     const uint64_t strides[1] = {(uint64_t)a.k_total * 2};
-    const uint32_t box[2] = {(uint32_t)BK, (uint32_t)WN};
+    const uint32_t box[2] = {(uint32_t)BK, (uint32_t)BN};
     if (int e = make_tmap_bf16(&tmW, a.w, 2, dims, strides, box, SW)) return e;
   }
 
   static SmemAttrCache smem_cache;
-  ADP_CUDA(ensure_dyn_smem(conv_gemm2_kernel<BN, SW, XF, EW, CG>, smem, smem_cache));
+  ADP_CUDA(ensure_dyn_smem(conv_gemm2_kernel<BN, SW, EW>, smem, smem_cache));
 
   p.out = static_cast<__nv_bfloat16*>(a.out);
   p.residual = static_cast<const __nv_bfloat16*>(a.residual);
@@ -767,62 +587,39 @@ static int launch_gemm2_ew(const adp_conv_gemm_args& a, cudaStream_t stream, int
   p.out_fp32 = a.out_fp32;
   p.ld_gate = a.ld_gate > 0 ? a.ld_gate : a.n_valid;
   p.n_tiles_n = a.phases * a.n_pad / BN;
-  p.total_tiles = (a.B * tiles_per_batch + CG - 1) / CG * p.n_tiles_n;   // pair tiles when CG == 2
+  p.total_tiles = a.B * tiles_per_batch * p.n_tiles_n;
   p.a_rows = a_rows;
-  p.dbg = g_debug[4];
-  p.early_w = g_debug[2];
-  p.gn_stats = a.gn_stats;
-  p.gn_gamma = a.gn_gamma;
-  p.gn_beta = a.gn_beta;
-  p.gn_eps = a.gn_eps;
-  p.gn_groups = a.gn_groups > 0 ? a.gn_groups : 1;
+  p.early_w = g_early_w;
 
-  // grid in units of CTA groups (single CTAs, or pairs)
-  const int slots = occ * num_sms() / CG;
+  const int slots = occ * num_sms();
   int grid = p.total_tiles < slots ? p.total_tiles : slots;
   p.tiles_per_cta = (p.total_tiles + grid - 1) / grid;
   grid = (p.total_tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
-  ADP_CUDA(launch_k_cluster(conv_gemm2_kernel<BN, SW, XF, EW, CG>, dim3(grid * CG),
-                            dim3(64 + 32 * EW + (XF ? 256 : 0)), smem, stream, CG, tmA, tmW, p));
+  ADP_CUDA(launch_k(conv_gemm2_kernel<BN, SW, EW>, dim3(grid), dim3(64 + 32 * EW), smem, stream, tmA, tmW, p));
   ADP_LAUNCH_CHECK();
   return 0;
 }
 
 template <int SW>
 static int dispatch_bn2(const adp_conv_gemm_args& a, int bn, cudaStream_t s) {
-  if (a.gn_stats) {
-    switch (bn) {
-      case 16: return launch_gemm2<16, SW, true>(a, s);
-      case 32: return launch_gemm2<32, SW, true>(a, s);
-      case 64: return launch_gemm2<64, SW, true>(a, s);
-      case 128: return launch_gemm2<128, SW, true>(a, s);
-      case 256: return launch_gemm2<256, SW, true>(a, s);
-    }
-  }
   switch (bn) {
-    case 16: return launch_gemm2<16, SW, false>(a, s);
-    case 32: return launch_gemm2<32, SW, false>(a, s);
-    case 64: return launch_gemm2<64, SW, false>(a, s);
-    case 128: return launch_gemm2<128, SW, false>(a, s);
-    case 256: return launch_gemm2<256, SW, false>(a, s);
+    case 16: return launch_gemm2<16, SW>(a, s);
+    case 32: return launch_gemm2<32, SW>(a, s);
+    case 64: return launch_gemm2<64, SW>(a, s);
+    case 128: return launch_gemm2<128, SW>(a, s);
+    case 256: return launch_gemm2<256, SW>(a, s);
   }
   return set_error("adp_conv_gemm: unsupported N tile %d", bn);
 }
 
 }  // namespace adp
 
-namespace adp { extern int g_mid_threads; }
-
 extern "C" int adp_debug_set(int key, int value) {
-  if (key == 8) {            // threads per block of the thin-level ConvBlock kernels (128 or 256)
-    if (value != 128 && value != 256) return adp::set_error("adp_debug_set: key 8 takes 128 or 256");
-    adp::g_mid_threads = value;
-    return 0;
+  switch (key) {
+    case 2: adp::g_early_w = value; return 0;
+    case 6: adp::g_pdl = value; return 0;
   }
-  if (key < 0 || key >= 8) return adp::set_error("adp_debug_set: bad key %d", key);
-  adp::g_debug[key] = value;
-  if (key == 6) adp::g_pdl = value;
-  return 0;
+  return adp::set_error("adp_debug_set: bad key %d (2 = early weight fetch, 6 = PDL)", key);
 }
 
 extern "C" int adp_conv_gemm(const adp_conv_gemm_args* args, adp_stream_t stream) {
@@ -854,11 +651,6 @@ extern "C" int adp_conv_gemm(const adp_conv_gemm_args* args, adp_stream_t stream
   }
   if (a.out_fp32) {
     ADP_CHECK(!a.residual && !a.stats, "adp_conv_gemm: out_fp32 excludes residual/stats");
-  }
-  if (a.gn_stats) {
-    ADP_CHECK(a.c_in <= 1024, "adp_conv_gemm: fused GroupNorm supports c_in <= 1024");
-    ADP_CHECK(a.gn_gamma && a.gn_beta && a.gn_groups > 0 && a.c_in % a.gn_groups == 0 && a.lda == a.c_in,
-              "adp_conv_gemm: fused GroupNorm needs gamma/beta, groups | c_in and a dense input");
   }
   if (a.stats) {
     ADP_CHECK(a.groups > 0 && a.groups <= kMaxGroups && a.n_valid % a.groups == 0,

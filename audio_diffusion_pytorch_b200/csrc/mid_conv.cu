@@ -33,12 +33,12 @@ __device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
-// NTH = threads per block.  256 threads x 2 blocks / SM or 128 threads x 4 blocks / SM (half-size
-// tiles): the same 16 warps per SM, but four independent barrier-separated phase streams instead
-// of two (selected by g_mid_threads, adp_debug_set(8, ..)).
-template <int C, int NTH>
+// 256 threads per block, 2 blocks per SM (128 x 4 half-size tiles measured no faster end to end,
+// DESIGN.md section 8)
+template <int C>
 struct MidCfg {
-  static constexpr int TB = (C == 32 ? 256 : 128) * NTH / 256;  // rows per tile
+  static constexpr int NTH = 256;                      // threads per block
+  static constexpr int TB = C == 32 ? 256 : 128;       // rows per tile
   static constexpr int TPR = NTH / TB;                 // staging threads per row
   static constexpr int RPW = TB / (NTH / 32);          // rows per warp in the MMA phase
   static constexpr int RS = C * 2 + 16;                // padded smem row stride of s_x (bytes)
@@ -63,10 +63,10 @@ struct MidCfg {
 // reduction.  (The first version ran the epilogue in the accumulator-fragment layout: 4-byte
 // stores, 4-byte shared-memory residual reads and a shuffle chain per fragment row made the
 // kernel issue/latency bound at 15-40 % of HBM bandwidth, profiles/r2_ncu_mid_conv64.txt.)
-template <int C, int NTH>
-__global__ void __launch_bounds__(NTH, 512 / NTH) mid_conv_kernel(const adp_narrow_conv_args a) {
-  using Cfg = MidCfg<C, NTH>;
-  constexpr int TB = Cfg::TB, TPR = Cfg::TPR, RS = Cfg::RS, WS = Cfg::WS, MB = Cfg::MB, NT = Cfg::NT;
+template <int C>
+__global__ void __launch_bounds__(256, 2) mid_conv_kernel(const adp_narrow_conv_args a) {
+  using Cfg = MidCfg<C>;
+  constexpr int NTH = Cfg::NTH, TB = Cfg::TB, TPR = Cfg::TPR, RS = Cfg::RS, WS = Cfg::WS, MB = Cfg::MB, NT = Cfg::NT;
   constexpr int OS = Cfg::OS, LPR = Cfg::LPR, ER = Cfg::ER, RPW = Cfg::RPW;
   pdl_launch_dependents();
   pdl_wait();
@@ -319,33 +319,28 @@ __global__ void __launch_bounds__(NTH, 512 / NTH) mid_conv_kernel(const adp_narr
   }
 }
 
-// 256: measured A/B on B200 (tools/time_mid_threads.py, L2 flushed): 128 x 4 is 5-6 % faster for
-// C = 32 at 16 batch rows, 7-8 % slower for C = 64 at 8, equal elsewhere; no change end to end
-int g_mid_threads = 256;
-
-template <int C, int NTH>
+template <int C>
 static int launch_mid(const adp_narrow_conv_args& a, cudaStream_t stream) {
-  using Cfg = MidCfg<C, NTH>;
+  using Cfg = MidCfg<C>;
   static SmemAttrCache smem_cache;
-  ADP_CUDA(ensure_dyn_smem(mid_conv_kernel<C, NTH>, (size_t)Cfg::SMEM, smem_cache));
+  ADP_CUDA(ensure_dyn_smem(mid_conv_kernel<C>, (size_t)Cfg::SMEM, smem_cache));
   int dev = 0, sms = 148, occ = 1;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mid_conv_kernel<C, NTH>, NTH, Cfg::SMEM) != cudaSuccess ||
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mid_conv_kernel<C>, Cfg::NTH, Cfg::SMEM) != cudaSuccess ||
       occ < 1)
     occ = 1;
   const int n_tiles = (a.T + Cfg::TB - 1) / Cfg::TB;
   int gx = (occ * sms) / a.B;               // one wave of persistent blocks
   if (gx < 1) gx = 1;
   if (gx > n_tiles) gx = n_tiles;
-  ADP_CUDA(launch_k(mid_conv_kernel<C, NTH>, dim3(gx, a.B), dim3(NTH), (size_t)Cfg::SMEM, stream, a));
+  ADP_CUDA(launch_k(mid_conv_kernel<C>, dim3(gx, a.B), dim3(Cfg::NTH), (size_t)Cfg::SMEM, stream, a));
   return 0;
 }
 
 int mid_conv(const adp_narrow_conv_args& a, cudaStream_t stream) {
-  const bool small = g_mid_threads == 128;
-  if (a.C == 32) return small ? launch_mid<32, 128>(a, stream) : launch_mid<32, 256>(a, stream);
-  if (a.C == 64) return small ? launch_mid<64, 128>(a, stream) : launch_mid<64, 256>(a, stream);
+  if (a.C == 32) return launch_mid<32>(a, stream);
+  if (a.C == 64) return launch_mid<64>(a, stream);
   return set_error("adp_narrow_conv: C=%d is not built (8, 32, 64)", a.C);
 }
 

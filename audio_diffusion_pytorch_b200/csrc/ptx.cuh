@@ -183,79 +183,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16
       : "memory");
 }
 
-// ------------------------------------------------------------- CTA pairs (cta_group::2)
-// Two CTAs of a cluster (same TPC) execute ONE tcgen05.mma of M = 256: each CTA holds its 128
-// rows of A and HALF of the B tile in its own shared memory and receives its 128 rows of D in
-// its own TMEM.  Only the leader (cluster rank 0) issues MMAs; completion is multicast to the
-// mbarriers at the same offset in both CTAs.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// every thread of every CTA in the cluster
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `smem_addr` (a shared::cta address) in the CTA of rank `rank`
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA loads of a CTA pair: data lands in THIS CTA's smem, completion bytes are signalled on the
-// mbarrier at `bar_cluster_addr` (the leader's full barrier, shared::cluster address)
-__device__ __forceinline__ void tma_load_2d_cg2(void* smem_dst, const CUtensorMap* m, uint32_t bar_cluster_addr,
-                                                int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4}], [%2];" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_cg2(void* smem_dst, const CUtensorMap* m, uint32_t bar_cluster_addr,
-                                                int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_cg2(uint32_t* smem_result, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                   smem_u32(smem_result)),
-               "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_cg2() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_cg2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void umma_bf16_cg2(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                              uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// completion of all MMAs issued so far -> one arrival on the mbarrier at this offset in EVERY
-// CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_cg2(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(cta_mask)
-      : "memory");
-}
-
 // ------------------------------------------------------------------------- descriptors
 // UMMA shared-memory matrix descriptor (sm_100): start>>4 [0,14) | LBO>>4 [16,30) |
 // SBO>>4 [32,46) | version=1 [46,48) | base_offset [49,52) | layout [61,64).

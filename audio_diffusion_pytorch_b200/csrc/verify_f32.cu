@@ -314,7 +314,7 @@ extern "C" int adp_f32_conv_gemm(const adp_conv_gemm_args* args, adp_stream_t st
   ADP_CHECK(args && args->a && args->w && args->out, "adp_f32_conv_gemm: null pointer");
   const adp_conv_gemm_args& a = *args;
   ADP_CHECK(a.B > 0 && a.T > 0 && a.c_in > 0 && a.n_valid > 0 && a.phases >= 1, "adp_f32_conv_gemm: bad sizes");
-  ADP_CHECK(!a.stats && !a.gn_stats, "adp_f32_conv_gemm: statistics / fused GroupNorm are separate passes");
+  ADP_CHECK(!a.stats, "adp_f32_conv_gemm: statistics are a separate pass");
   ADP_CHECK(a.up_factor <= 1 || a.phases == a.up_factor, "adp_f32_conv_gemm: phases != up_factor");
   ADP_CHECK(a.up_factor > 1 || (a.ntaps >= 1 && a.ntaps <= 3 && a.phases == 1), "adp_f32_conv_gemm: taps");
   ADP_CUDA(launch_k(f32_conv_gemm_kernel, dim3(f32_grid(static_cast<int64_t>(a.B) * a.T * a.phases * a.n_valid)),

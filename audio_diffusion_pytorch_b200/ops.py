@@ -156,8 +156,7 @@ def pack_upsample_conv(w: Tensor, f: int) -> Tensor:
 def conv_gemm(a: Tensor, w: Tensor, out: Tensor, *, c_in: int, n_valid: int,
               taps: Sequence[int] = (0,), up_factor: int = 0, bias: Optional[Tensor] = None,
               residual: Optional[Tensor] = None, gate: Optional[Tensor] = None,
-              stats: Optional[Tensor] = None, groups: int = 8, block_n: int = 0,
-              gn: Optional[tuple] = None) -> Tensor:
+              stats: Optional[Tensor] = None, groups: int = 8, block_n: int = 0) -> Tensor:
     """a: bf16 [B, T, lda]; w: packed bf16 [phases*n_pad, k_total]; out: [B, T, ldo]."""
     B, T, lda = a.shape
     phases = up_factor if up_factor > 1 else 1
@@ -173,21 +172,18 @@ def conv_gemm(a: Tensor, w: Tensor, out: Tensor, *, c_in: int, n_valid: int,
     args.up_factor, args.groups, args.block_n = up_factor, groups, block_n
     args.out_fp32 = 1 if out.dtype == torch.float32 else 0
     args.ld_gate = 0 if gate is None else gate.stride(0)
-    if gn is not None:      # (stats_of_a, gamma, beta, groups, eps): a := SiLU(GroupNorm(a)) fused
-        args.gn_stats, args.gn_gamma, args.gn_beta = gn[0].data_ptr(), gn[1].data_ptr(), gn[2].data_ptr()
-        args.gn_groups, args.gn_eps = gn[3], gn[4]
 
     def meta():
         rows = B * T
         tap_sum = len(taps) if up_factor <= 1 else (4 if up_factor == 2 else up_factor + 2)
-        kind = ("up%d" % up_factor if up_factor > 1 else "k%d" % len(taps)) + ("+gn" if gn is not None else "")
+        kind = "up%d" % up_factor if up_factor > 1 else "k%d" % len(taps)
         flops = 2.0 * rows * c_in * n_valid * tap_sum
         nbytes = rows * c_in * 2 + w.shape[0] * min(w.shape[1], tap_sum * c_in) * 2 \
             + rows * phases * n_valid * out.element_size() * (2 if residual is not None else 1)
         return f"conv_gemm[{kind} M={rows} K={c_in} N={n_valid}x{phases}]", flops, nbytes
 
     if a.dtype == torch.float32:       # fp32 verification mode (csrc/verify_f32.cu)
-        assert w.dtype == torch.float32 and out.dtype == torch.float32 and gn is None
+        assert w.dtype == torch.float32 and out.dtype == torch.float32
         assert residual is None or residual.dtype == torch.float32
         args.stats, args.out_fp32 = None, 0
         _launch(lambda: _lib.lib().adp_f32_conv_gemm(C.byref(args), _stream()), "adp_f32_conv_gemm", meta)

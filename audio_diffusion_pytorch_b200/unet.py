@@ -240,11 +240,6 @@ class B200UNet(nn.Module):
         self._storage_sig = None
         self._repack_graph = None
         self.use_cuda_graph = True
-        # GroupNorm+SiLU applied inside the conv GEMM by transform warps (adp_conv_gemm gn_*).
-        # Verified bit-compatible with the two-kernel path but measured SLOWER on the README
-        # config (6.85 vs 6.0 ms / evaluation, profiles/r1_gn_fusion.txt): every N tile repeats
-        # the transform of its A rows, so it only pays for N <= BN.  Off by default.
-        self.fuse_groupnorm = False
         # C = 32 / 64 ConvBlocks as ONE fused kernel (GroupNorm+SiLU -> conv3 -> +res -> LN/FiLM ->
         # statistics, csrc/mid_conv.cu) instead of three: those levels are HBM-bound
         self.fuse_thin_levels = True
@@ -692,27 +687,18 @@ class B200UNet(nn.Module):
                     # use_modulation=False: the ResnetItem's output IS the item's output, so its
                     # GroupNorm statistics come out of conv2's epilogue
                     rs = None if mod else mod_stats
-                    if self.fuse_groupnorm:
-                        # ConvBlock = ONE kernel: GroupNorm+SiLU applied to the smem A tile
-                        plan.add(lambda x=x, h=h, s=x_stats, hs=h_stats, ip=ip: ops.conv_gemm(
-                            x, ip["w1"], h, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b1"], stats=hs,
-                            groups=G, gn=(s, ip["gn1"][0], ip["gn1"][1], G, self.GN_EPS)))
-                        plan.add(lambda x=x, h=h, r=r, hs=h_stats, ip=ip, rs=rs: ops.conv_gemm(
-                            h, ip["w2"], r, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b2"], residual=x,
-                            stats=rs, groups=G, gn=(hs, ip["gn2"][0], ip["gn2"][1], G, self.GN_EPS)))
-                    else:
-                        a = pool.get(Bh, Tl, C)
-                        plan.add(lambda x=x, a=a, s=x_stats, ip=ip: ops.gn_silu(
-                            x, a, s, ip["gn1"][0], ip["gn1"][1], G, self.GN_EPS))
-                        plan.add(lambda a=a, h=h, hs=h_stats, ip=ip: ops.conv_gemm(
-                            a, ip["w1"], h, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b1"], stats=hs,
-                            groups=G))
-                        plan.add(lambda a=a, h=h, hs=h_stats, ip=ip: ops.gn_silu(
-                            h, a, hs, ip["gn2"][0], ip["gn2"][1], G, self.GN_EPS))
-                        plan.add(lambda x=x, a=a, r=r, ip=ip, rs=rs: ops.conv_gemm(
-                            a, ip["w2"], r, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b2"], residual=x,
-                            stats=rs, groups=G))
-                        pool.put(a)
+                    a = pool.get(Bh, Tl, C)
+                    plan.add(lambda x=x, a=a, s=x_stats, ip=ip: ops.gn_silu(
+                        x, a, s, ip["gn1"][0], ip["gn1"][1], G, self.GN_EPS))
+                    plan.add(lambda a=a, h=h, hs=h_stats, ip=ip: ops.conv_gemm(
+                        a, ip["w1"], h, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b1"], stats=hs,
+                        groups=G))
+                    plan.add(lambda a=a, h=h, hs=h_stats, ip=ip: ops.gn_silu(
+                        h, a, hs, ip["gn2"][0], ip["gn2"][1], G, self.GN_EPS))
+                    plan.add(lambda x=x, a=a, r=r, ip=ip, rs=rs: ops.conv_gemm(
+                        a, ip["w2"], r, c_in=C, n_valid=C, taps=(-1, 0, 1), bias=ip["b2"], residual=x,
+                        stats=rs, groups=G))
+                    pool.put(a)
                     xn_first = pool.get(Bh, Tl, C) if ((has_att or has_cross) and not has_inj and mod) else None
                     if mod:
                         # Modulation and the following attention pre-norm in ONE pass over the rows

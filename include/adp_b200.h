@@ -35,8 +35,11 @@ int adp_version(void);
 const char* adp_last_error(void);
 /* 0 iff the current CUDA device is compute capability 10.x (B200). */
 int adp_device_check(void);
-/* Diagnostic switches for A/B runs (key 0: GEMM implementation 2=persistent 1=v1; key 1: one
- * A box for all taps; key 2: descriptor base-offset mode).  Not part of the hot path. */
+/* Process-wide launch switches, read when a kernel is launched (or captured into a graph):
+ *  key 2: 1 = adp_conv_gemm may fetch its weights before waiting for the preceding kernel (valid
+ *         while no preceding kernel writes them, e.g. in an inference graph); default 0.
+ *  key 6: 1 = launch with programmatic dependent launch (PDL); 0 = plain stream order; default 1.
+ * Any other key is an error. */
 int adp_debug_set(int key, int value);
 
 /* ---------------------------------------------------------------------------------------
@@ -73,13 +76,6 @@ typedef struct adp_conv_gemm_args {
   int32_t block_n;      /* N tile override (16..256), 0 = auto      */
   int32_t out_fp32;     /* 1: `out` is fp32 [B][T][ldo] (conditioning projections); no residual */
   int32_t ld_gate;      /* row pitch of gate in elements (multiple of 4); 0 = n_valid */
-  /* optional fused prologue: a := SiLU(GroupNorm(a)) applied to the smem tile before the MMAs
-   * (a_unet ConvBlock's GroupNorm + SiLU); gn_stats = fp64 [B][gn_groups][2] of `a`. */
-  const double* gn_stats;
-  const float* gn_gamma;
-  const float* gn_beta;
-  float gn_eps;
-  int32_t gn_groups;
 } adp_conv_gemm_args;
 int adp_conv_gemm(const adp_conv_gemm_args* args, adp_stream_t stream);
 

@@ -98,25 +98,6 @@ def test_unconditional_net_and_sampler_vs_golden(adp, oracle_port, golden_dir):
     model.net.cond_table_rows = 4096
 
 
-def test_fused_groupnorm_gemm_path_matches(adp, oracle_port, golden_dir):
-    """Optional path (B200UNet.fuse_groupnorm): GroupNorm+SiLU applied inside the conv GEMM."""
-    g = load(golden_dir, "tiny_unconditional.npz")
-    torch.manual_seed(0)
-    ref = oracle_port.DiffusionModelPort(**TINY)
-    model = adp.DiffusionModel(net_t=adp.UNetV0, **TINY).to(DEV)
-    model.net.load_reference_parameters(ref.net)
-    x, sigma = t(g["x"]), t(g["sigma"])
-    v_two_kernel = model.net(x, sigma).clone()
-    model.net.fuse_groupnorm = True
-    model.net._plans.clear()
-    for call in range(3):
-        v = model.net(x, sigma)
-        check(v, torch.from_numpy(g["v"]), x, f"fused-GN forward (call {call})")
-    e = rel_l2(v, v_two_kernel.cpu())
-    print(f"fused-GN vs two-kernel path: rel-L2 {e:.3e}")
-    assert e <= 1e-4
-
-
 def test_text_cfg_vs_golden(adp, oracle_port, golden_dir):
     g = load(golden_dir, "tiny_text_cfg.npz")
     torch.manual_seed(0)

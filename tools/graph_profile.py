@@ -91,7 +91,6 @@ def main():
         x = torch.randn(w["batch"], 2, 2 ** 18, device="cuda")
         if cfg == "cfg3":
             kw = dict(embedding=torch.randn(w["batch"], 64, 768, device="cuda"), embedding_scale=5.0)
-    model.net.fuse_groupnorm = os.environ.get("ADP_FUSE_GN", "0") == "1"
     for _ in range(2):
         model.sample(x, num_steps=3, **kw)          # eager + capture
     plan = next(p for k, p in model.net._plans.items() if len(k) > 4 and k[4] == "sample")

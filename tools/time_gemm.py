@@ -1,10 +1,10 @@
-"""Timing of adp_conv_gemm variants: 40 launches captured in a CUDA graph, replayed (device time only).
-usage: python tools/time_gemm.py"""
+"""Graph-timed adp_conv_gemm on the README net's GEMM shapes at B=8, for every N tile that divides N
+(bias + residual + GroupNorm statistics, as the conv3 of a ResnetItem runs).  20 launches captured
+in a CUDA graph, replayed (device time only).  usage: python tools/time_gemm.py"""
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from audio_diffusion_pytorch_b200 import _lib, ops
-L = _lib.lib()
+from audio_diffusion_pytorch_b200 import ops
 dev = "cuda"
 
 def run(M, K, N, taps, bn, res=True, stats=False, B=8, reps=20):
@@ -32,20 +32,19 @@ def run(M, K, N, taps, bn, res=True, stats=False, B=8, reps=20):
     return us, fl / us / 1e6
 
 if __name__ == "__main__":
-    shapes = [("L1 conv3", 524288, 32, 32, 3), ("L7 conv3", 2048, 1024, 1024, 3), ("L8 conv3", 1024, 1024, 1024, 3), ("L5 conv3", 8192, 512, 512, 3),
-              ("L4 conv3", 16384, 256, 256, 3), ("L3 conv3", 32768, 128, 128, 3), ("L2 conv3", 131072, 64, 64, 3),
-              ("L7 qkv", 2048, 1024, 1536, 1), ("L5 qkv", 8192, 512, 1536, 1)]
-    modes = [("v1", 1, 1, 0, 0), ("v3", 2, 1, 0, 0), ("noMMA", 2, 1, 0, 1), ("noLOAD", 2, 1, 0, 2), ("neither", 2, 1, 0, 3)]
+    shapes = [("L1 conv3", 524288, 32, 32, 3), ("L2 conv3", 131072, 64, 64, 3), ("L3 conv3", 32768, 128, 128, 3),
+              ("L4 conv3", 16384, 256, 256, 3), ("L5 conv3", 8192, 512, 512, 3), ("L6 conv3", 4096, 512, 512, 3),
+              ("L7 conv3", 2048, 1024, 1024, 3), ("L8 conv3", 1024, 1024, 1024, 3),
+              ("L7 qkv", 2048, 1024, 1536, 1), ("L5 qkv", 8192, 512, 1536, 1), ("L7 out", 2048, 512, 1024, 1),
+              ("L5 out", 8192, 512, 512, 1)]
     for name, M, K, N, taps in shapes:
-        for bn in (32, 64, 128):
-            if N % max(bn, 16): continue
-            if bn > N: continue
-            row = []
-            for mname, impl, single, occ, dbg in modes:
-                L.adp_debug_set(0, impl); L.adp_debug_set(1, single); L.adp_debug_set(3, occ); L.adp_debug_set(4, dbg)
-                try:
-                    us, tf = run(M, K, N, taps, bn, res=False, stats=False)
-                    row.append(f"{mname}: {us:6.1f}us {tf:5.0f}TF")
-                except Exception as e:
-                    row.append(f"{mname}: ERR {str(e)[:40]}")
-            print(f"{name:9s} bn={bn:3d} | " + " | ".join(row), flush=True)
+        row = []
+        for bn in (32, 64, 128, 256):
+            if N % bn:
+                continue
+            try:
+                us, tf = run(M, K, N, taps, bn, res=True, stats=True)
+                row.append(f"bn{bn}: {us:6.1f}us {tf:5.0f}TF")
+            except Exception as e:
+                row.append(f"bn{bn}: ERR {str(e)[:30]}")
+        print(f"{name:9s} | " + " | ".join(row), flush=True)
